@@ -2,6 +2,7 @@
 """bench.py — candidate-sites/sec of the Clair3 network forward on B200 (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workloads pileup,fa,fa_dwell,cascade]
+                    [--dump-outputs DIR]
 
 ONE command measures the whole metric and prints ONE JSON line.  The top-level ``value`` / ``e2e`` / ``roofline`` are the
 pileup network on BASELINE.json configs[1] (the configuration the metric is quoted on); ``workloads`` carries one
@@ -16,24 +17,29 @@ sub-record per configuration:
     pileup_counts  SURVEY.md 8f row N4: the pileup feature counter (calculate_clair3_pileup, src/clair3_pileup.c:142-476) on
               decoded alignment records, aligned bases/s (its own metric; HBM-bound integer work)          weak
 
-A *step* is one forward of the hot path over one synthetic candidate-site batch.  Every timed region issues the K steps
-``repeats`` times back to back so that it lasts >= 2 s whatever K is (``timed_region_s``, ``repeats`` in the record;
-``ms_per_step`` = region / (K * repeats)); W warm-up steps precede it.  Steps go round-robin over a few CUDA streams of ONE
-model (each stream owns an activation workspace); device-resident inputs are rotated over > 126 MB of distinct batches so
-no step re-reads its input from L2; regions are bracketed by barrier + synchronize, timed with CUDA events, max over ranks;
-``nvidia-smi`` clocks are sampled every 100 ms DURING each region.  ``e2e`` is the same metric through the module API with
-pinned HOST input and HOST output (H2D and D2H inside the timed region): pipelined (``forward_async`` over the streams),
-through the ``predict_stream`` helper, and synchronous per step (the reference's ``_torch_predict`` shape).
+A *step* is one forward of the hot path over one synthetic candidate-site batch (for ``cascade``: one pass over all its
+sites).  Every timed region is exactly K steps (``timed_region_s``; ``ms_per_step`` = region / K); W warm-up steps precede
+it.  A small K times pipeline fill and drain as much as the steady state: pass a K whose region lasts seconds for a rate.
+Steps go round-robin over a few CUDA streams of ONE model (each stream owns an activation workspace); device-resident
+inputs are rotated over > 126 MB of distinct batches so no step re-reads its input from L2; regions are bracketed by
+barrier + synchronize, timed with CUDA events, max over ranks; ``nvidia-smi`` clocks are sampled every 100 ms DURING each
+region.  ``e2e`` is the same metric through the module API with pinned HOST input and HOST output (H2D and D2H inside the
+timed region): pipelined (``forward_async`` over the streams), through the ``predict_stream`` helper, and synchronous per
+step (the reference's ``_torch_predict`` shape).
 
 N > 1: one process per GPU (torchrun), one NCCL broadcast of the packed weight images from rank 0 before timing
 (``c3b_bcast_weights``), no data-path collective.
 
 ``--impl reference`` times the reference's own CPU implementation of the same steps (torch CPU ops, all host threads)
 through ``oracle/torch_port.py`` (the Python reference cannot travel to the GPU box; see DESIGN.md).
+
+``--dump-outputs DIR`` writes, after the timed regions, what the last timed step of each workload returned to its caller as
+``DIR/<workload>[_<array>].npy`` (float32 probabilities; integer counts as float64, exact), so that two builds run with the
+same arguments - hence the same seeded inputs - can be compared output for output.  Outputs larger than a few MB are a fixed,
+seeded sample of rows (``*_rows.npy`` holds the row indices); the whole dump stays under 64 MB.
 """
 import argparse
 import json
-import math
 import os
 import subprocess
 import sys
@@ -46,10 +52,14 @@ import torch
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+# the tree may be read-only: neither this process nor its CPU-baseline workers write bytecode caches into it
+sys.dont_write_bytecode = True
+os.environ["PYTHONDONTWRITEBYTECODE"] = "1"
 
 from clair3_b200 import synth  # noqa: E402
 
-MIN_REGION_S = 2.0
+DUMP_MAX_BYTES = 64 << 20
+DUMP_SAMPLE_ROWS = 65536
 
 # algorithmic FLOPs per site (SURVEY.md 8d) and per tensor-core kernel (2*M*N*K of the layer shapes, clair3/model.py:96-110, 317-344)
 WORKLOADS = {
@@ -345,6 +355,7 @@ class Ctx:
         self.args, self.rank, self.world, self.device, self.sampler = args, rank, world, device, sampler
         self.streams = [torch.cuda.Stream(device) for _ in range(max(1, args.streams))]
         self.main = torch.cuda.current_stream(device)
+        self.dump = {} if args.dump_outputs and rank == 0 else None     # name -> the last timed step's output (host array)
 
     def barrier(self):
         if self.world > 1:
@@ -383,22 +394,23 @@ class Ctx:
         self.barrier()
         return ms, clocks
 
-    def calibrated(self, issue, steps, est_calls=None):
-        """Run `steps` once untimed-for-the-record to estimate the step time, then a region of `repeats` x `steps` calls that
-        lasts >= MIN_REGION_S.  Returns dict(ms, repeats, clocks)."""
-        n0 = est_calls or max(steps, 2 * len(self.streams))
-        ms0, _ = self.timed(issue, n0)
-        per_call = max(ms0 / n0, 1e-4)
-        repeats = max(1, int(math.ceil(MIN_REGION_S * 1e3 * 1.1 / (per_call * steps))))
-        for _ in range(3):
-            if self.world > 1:
-                repeats = int(self.max_over_ranks([repeats])[0])
-            ms, clocks = self.timed(issue, steps * repeats)
-            if ms >= MIN_REGION_S * 1e3 or MIN_REGION_S <= 0:
-                break
-            # the estimate ran at burst clocks and the long region at the power-capped sustained ones: scale up and re-measure
-            repeats = int(math.ceil(repeats * MIN_REGION_S * 1e3 * 1.15 / max(ms, 1e-3)))
-        return {"ms": ms, "repeats": repeats, "clocks": clocks}
+
+def sample_rows(n, seed=0):
+    """Indices of a fixed, seeded, sorted sample of DUMP_SAMPLE_ROWS of n rows (all rows when n is not larger)."""
+    if n <= DUMP_SAMPLE_ROWS:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(seed).choice(n, DUMP_SAMPLE_ROWS, replace=False))
+
+
+def dump_outputs(dirname, arrays):
+    """Write name -> array as DIR/<name>.npy: floating outputs as float32, integer ones as float64 (exact below 2**53)."""
+    out = {k: np.ascontiguousarray(a, dtype=np.float32 if a.dtype.kind == "f" else np.float64) for k, a in arrays.items()}
+    total = sum(a.nbytes for a in out.values())
+    if total > DUMP_MAX_BYTES:
+        raise SystemExit("--dump-outputs: %d bytes exceed the %d-byte limit" % (total, DUMP_MAX_BYTES))
+    os.makedirs(dirname, exist_ok=True)
+    for k, a in out.items():
+        np.save(os.path.join(dirname, k + ".npy"), a)
 
 
 def parity_spot_check(model, w, x):
@@ -512,12 +524,13 @@ def run_forward_workload(ctx, wname, model):
     torch.cuda.synchronize(dev)
     issue_dev(args.warmup)                                            # W warm-up steps
     launches0 = model.launch_count
-    r = ctx.calibrated(issue_dev, K)
-    est = max(K, 2 * n_streams)                                       # calls of the calibration pass before the final region
-    launches = (model.launch_count - launches0) * (K * r["repeats"]) // (K * r["repeats"] + est)   # the final region's share
-    value = b * K * r["repeats"] * ctx.world / (r["ms"] * 1e-3)
-    rec = {"value": value, "unit": "sites/s", "scaling": "weak", "steps": K, "repeats": r["repeats"],
-           "timed_region_s": r["ms"] * 1e-3, "ms_per_step": r["ms"] / (K * r["repeats"]), "clocks": r["clocks"],
+    ms, clocks = ctx.timed(issue_dev, K)
+    launches = model.launch_count - launches0
+    if ctx.dump is not None:
+        ctx.dump[wname] = ys_dev[(counter[0] - 1) % len(ys_dev)].cpu().numpy()
+    value = b * K * ctx.world / (ms * 1e-3)
+    rec = {"value": value, "unit": "sites/s", "scaling": "weak", "steps": K,
+           "timed_region_s": ms * 1e-3, "ms_per_step": ms / K, "clocks": clocks,
            "gpu_launches": int(launches), "parity_max_abs_dp": parity, "config": config_of(wname),
            "run": {"streams_in_flight": n_streams, "lstm_subtile_sites": (args.lstm_tile or "auto (64 stream-ordered / 16 synchronous)") if w["kind"] == "pileup" else None,
                    "l2_policy": "inputs rotated over %d distinct device-resident batches (> 126 MB L2)" % pool}}
@@ -537,11 +550,11 @@ def run_forward_workload(ctx, wname, model):
 
     issue_e2e(2 * n_streams)
     torch.cuda.synchronize(dev)
-    re = ctx.calibrated(issue_e2e, K)
+    e2e_ms, e2e_clocks = ctx.timed(issue_e2e, K)
     last = (ecount[0] - 1)
     ref_y = model(xs_pin[last % len(xs_pin)])                         # the last pipelined result must equal a sync call
     assert float((ref_y - ys_pin[last % n_streams]).abs().max()) < 1e-4
-    e2e_value = b * K * re["repeats"] * ctx.world / (re["ms"] * 1e-3)
+    e2e_value = b * K * ctx.world / (e2e_ms * 1e-3)
 
     # (b) the predict_stream helper (what a `_torch_predict`-shaped caller switches to)
     def run_stream(n):
@@ -551,10 +564,9 @@ def run_forward_workload(ctx, wname, model):
             cnt += len(y)
         return cnt
     run_stream(2 * n_streams)
-    n_ps = max(K, int(K * re["repeats"] // 2)) if MIN_REGION_S > 0 else K
     ctx.barrier()
     t0 = time.perf_counter()
-    run_stream(n_ps)
+    run_stream(K)
     torch.cuda.synchronize(dev)
     ps_ms = ctx.max_over_ranks([(time.perf_counter() - t0) * 1e3])[0]
 
@@ -562,11 +574,10 @@ def run_forward_workload(ctx, wname, model):
     for i in range(3):
         model(xs_pin[i % len(xs_pin)])
     torch.cuda.synchronize(dev)
-    n_sync = max(K, int(0.5e3 / max(re["ms"] / (K * re["repeats"]) * 4, 1e-3))) if MIN_REGION_S > 0 else K       # ~0.5+ s
     ctx.barrier()
     s0, s1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     s0.record()
-    for i in range(n_sync):
+    for i in range(K):
         y_host = model(xs_pin[i % len(xs_pin)])
     s1.record()
     torch.cuda.synchronize(dev)
@@ -593,25 +604,25 @@ def run_forward_workload(ctx, wname, model):
 
         issue_win(2 * n_streams)
         torch.cuda.synchronize(dev)
-        rw = ctx.calibrated(issue_win, K)
-        win = {"value": b * K * rw["repeats"] * ctx.world / (rw["ms"] * 1e-3), "unit": "sites/s", "steps": K, "repeats": rw["repeats"],
-               "timed_region_s": rw["ms"] * 1e-3, "h2d_bytes_per_step": n_cols * 18 * 8 + b * 8,
+        win_ms, _ = ctx.timed(issue_win, K)
+        win = {"value": b * K * ctx.world / (win_ms * 1e-3), "unit": "sites/s", "steps": K,
+               "timed_region_s": win_ms * 1e-3, "h2d_bytes_per_step": n_cols * 18 * 8 + b * 8,
                "mode": "Clair3_P.forward_windows(pinned int64 column matrix [%d,18], pinned window starts) pipelined over %d streams: "
                        "the 33-row windows are gathered on the GPU (candidates every %dth column)" % (n_cols, n_streams, stride_cols)}
     kind = "P" if w["kind"] == "pileup" else "F"
     rec["e2e"] = {"value": e2e_value, "unit": "sites/s", "h2d_bytes_per_step": in_bytes, "d2h_bytes_per_step": b * model.out_dim * 4,
-                  "steps": K, "repeats": re["repeats"], "timed_region_s": re["ms"] * 1e-3, "clocks": re["clocks"],
+                  "steps": K, "timed_region_s": e2e_ms * 1e-3, "clocks": e2e_clocks,
                   "mode": "Clair3_%s.forward_async(pinned host x, pinned host y) pipelined over %d streams (H2D + kernels + D2H "
                           "stream-ordered per step, one synchronise at the end)" % (kind, n_streams),
-                  "predict_stream": {"value": b * n_ps * ctx.world / (ps_ms * 1e-3), "unit": "sites/s", "steps": n_ps,
+                  "predict_stream": {"value": b * K * ctx.world / (ps_ms * 1e-3), "unit": "sites/s", "steps": K,
                                      "mode": "for Y in model.predict_stream(batches): in-order numpy results, %d batches in flight "
                                              "(host wall clock, includes the per-batch result copy)" % n_streams},
-                  "synchronous_per_step": {"value": b * n_sync * ctx.world / (sync_ms * 1e-3), "unit": "sites/s", "steps": n_sync,
+                  "synchronous_per_step": {"value": b * K * ctx.world / (sync_ms * 1e-3), "unit": "sites/s", "steps": K,
                                            "mode": "y = model(x_pinned): H2D, forward, D2H, stream sync every step (the _torch_predict shape)"}}
     if win:
         rec["e2e"]["forward_windows"] = win
     if ctx.rank == 0:
-        rec["kernels"], rec["roofline"] = profile_kernels(ctx, model, w, xs_dev, value, r["clocks"])
+        rec["kernels"], rec["roofline"] = profile_kernels(ctx, model, w, xs_dev, value, clocks)
     del xs_dev, ys_dev
     torch.cuda.empty_cache()
     return rec
@@ -626,10 +637,11 @@ def run_cascade(ctx, model_p, model_f):
     wp, wf = WORKLOADS["pileup"], WORKLOADS["fa"]
     pool_p = [torch.from_numpy(x).pin_memory() for x in make_inputs(wp, 64, seed=5000 + 977 * ctx.rank)]      # 156 MB
     pool_f = [torch.from_numpy(x).pin_memory() for x in make_inputs(wf, 24, seed=6000 + 977 * ctx.rank)]      # 144 MB
-    yp = [torch.empty((wp["batch"], model_p.out_dim), dtype=torch.float32).pin_memory() for _ in range(n_streams)]
-    yf = [torch.empty((wf["batch"], model_f.out_dim), dtype=torch.float32).pin_memory() for _ in range(n_streams)]
     lo_p, hi_p = sharding.site_range(CASCADE_PILEUP_SITES, ctx.rank, ctx.world)
     lo_f, hi_f = sharding.site_range(CASCADE_FA_SITES, ctx.rank, ctx.world)
+    # one pinned row per site of the rank's range: a pass leaves every result of the pass for its caller
+    yp = torch.empty((hi_p - lo_p, model_p.out_dim), dtype=torch.float32).pin_memory()
+    yf = torch.empty((hi_f - lo_f, model_f.out_dim), dtype=torch.float32).pin_memory()
 
     def batches(lo, hi, b):
         out = []
@@ -644,7 +656,7 @@ def run_cascade(ctx, model_p, model_f):
         for i, n in enumerate(bp_list):
             st = ctx.streams[i % n_streams]
             with torch.cuda.stream(st):
-                model_p.forward_async(pool_p[i % len(pool_p)][:n], yp[i % n_streams][:n])
+                model_p.forward_async(pool_p[i % len(pool_p)][:n], yp[i * wp["batch"]:i * wp["batch"] + n])
         # phase boundary: full-alignment candidates come out of the pileup calls, so the second phase starts after the first
         evs = []
         for st in ctx.streams:
@@ -657,29 +669,26 @@ def run_cascade(ctx, model_p, model_f):
         for i, n in enumerate(bf_list):
             st = ctx.streams[i % n_streams]
             with torch.cuda.stream(st):
-                model_f.forward_async(pool_f[i % len(pool_f)][:n], yf[i % n_streams][:n])
+                model_f.forward_async(pool_f[i % len(pool_f)][:n], yf[i * wf["batch"]:i * wf["batch"] + n])
 
     def issue(passes):
         for _ in range(passes):
             one_pass()
 
-    issue(1)                       # warm-up pass (workspaces, pinned pages)
+    issue(args.warmup)             # warm-up passes (workspaces, pinned pages)
     torch.cuda.synchronize(dev)
-    ms0, _ = ctx.timed(issue, 1)
-    passes = max(1, int(math.ceil(MIN_REGION_S * 1e3 * 1.1 / ms0)))
-    for _ in range(3):
-        if ctx.world > 1:
-            passes = int(ctx.max_over_ranks([passes])[0])
-        ms, clocks = ctx.timed(issue, passes)
-        if ms >= MIN_REGION_S * 1e3 or MIN_REGION_S <= 0:
-            break
-        passes = int(math.ceil(passes * MIN_REGION_S * 1e3 * 1.15 / max(ms, 1e-3)))
+    passes = args.steps
+    ms, clocks = ctx.timed(issue, passes)
+    if ctx.dump is not None:
+        rp, rf = sample_rows(len(yp)), sample_rows(len(yf))
+        ctx.dump.update({"cascade_pileup": yp.numpy()[rp], "cascade_pileup_rows": rp,
+                         "cascade_full_alignment": yf.numpy()[rf], "cascade_full_alignment_rows": rf})
     total = CASCADE_PILEUP_SITES + CASCADE_FA_SITES
     value = total * passes / (ms * 1e-3)
     h2d = (hi_p - lo_p) * site_bytes(wp) + (hi_f - lo_f) * site_bytes(wf)
     d2h = (hi_p - lo_p) * model_p.out_dim * 4 + (hi_f - lo_f) * model_f.out_dim * 4
-    rec = {"value": value, "unit": "sites/s", "scaling": "strong", "passes": passes, "repeats": passes,
-           "steps": len(bp_list) + len(bf_list), "timed_region_s": ms * 1e-3, "ms_per_pass": ms / passes, "clocks": clocks,
+    rec = {"value": value, "unit": "sites/s", "scaling": "strong", "passes": passes, "steps": passes,
+           "calls_per_pass": len(bp_list) + len(bf_list), "timed_region_s": ms * 1e-3, "ms_per_pass": ms / passes, "clocks": clocks,
            "sites_per_pass": {"pileup": CASCADE_PILEUP_SITES, "full_alignment": CASCADE_FA_SITES},
            "rank0_range": {"pileup": [lo_p, hi_p], "full_alignment": [lo_f, hi_f]} if ctx.rank == 0 else None,
            "config": config_of("cascade"),
@@ -741,8 +750,14 @@ def run_pileup_counts(ctx):
     issue_dev(2 * n_ctr)
     torch.cuda.synchronize(dev)
     issue_dev(args.warmup)
-    r = ctx.calibrated(issue_dev, K)
-    value = bases * K * r["repeats"] * ctx.world / (r["ms"] * 1e-3)
+    ms, clocks = ctx.timed(issue_dev, K)
+    value = bases * K * ctx.world / (ms * 1e-3)
+    if ctx.dump is not None:                      # what a caller fetches after the last timed count
+        got = counters[(cnt[0] - 1) % n_ctr].fetch()
+        rows = sample_rows(len(got["major"]))
+        ctx.dump.update({"pileup_counts_matrix": got["matrix"][rows], "pileup_counts_major": got["major"][rows],
+                         "pileup_counts_stats": got["stats"][rows], "pileup_counts_rows": rows,
+                         "pileup_counts_cand_cols": got["cand_cols"], "pileup_counts_cand_ok": got["cand_ok"]})
 
     # e2e: pinned host records in, results out, synchronous per call (the shape of the reference's per-chunk call)
     pin = pc.BamRecords(**{k: torch.from_numpy(getattr(host, k).view({"uint16": np.int16, "uint32": np.int32}.get(getattr(host, k).dtype.name, getattr(host, k).dtype))).pin_memory().numpy().view(getattr(host, k).dtype)
@@ -756,8 +771,8 @@ def run_pileup_counts(ctx):
         ecnt[0] += n
 
     issue_e2e(2)
-    re = ctx.calibrated(issue_e2e, max(2, K // 4), est_calls=2)
-    e2e_value = bases * max(2, K // 4) * re["repeats"] * ctx.world / (re["ms"] * 1e-3)
+    e2e_ms, _ = ctx.timed(issue_e2e, K)
+    e2e_value = bases * K * ctx.world / (e2e_ms * 1e-3)
     h2d = host.nbytes() + len(ref)
     d2h = n_cols * (18 * 8 + 8 + 24) + n_cand * 9
     pk = peaks()
@@ -771,15 +786,15 @@ def run_pileup_counts(ctx):
             traffic = ent["dram_bytes_per_launch"]
     except (OSError, ValueError, KeyError):
         pass
-    out = {"metric": "aligned-bases/sec", "value": value, "unit": "bases/s", "scaling": "weak", "steps": K, "repeats": r["repeats"],
-           "timed_region_s": r["ms"] * 1e-3, "ms_per_step": r["ms"] / (K * r["repeats"]), "clocks": r["clocks"],
-           "columns_per_s": n_cols * K * r["repeats"] * ctx.world / (r["ms"] * 1e-3),
-           "gpu_launches": int(launches_per_call * K * r["repeats"]), "parity": "bit-exact vs oracle/pileup_oracle.c on the first 65536 columns of the bench input",
+    out = {"metric": "aligned-bases/sec", "value": value, "unit": "bases/s", "scaling": "weak", "steps": K,
+           "timed_region_s": ms * 1e-3, "ms_per_step": ms / K, "clocks": clocks,
+           "columns_per_s": n_cols * K * ctx.world / (ms * 1e-3),
+           "gpu_launches": int(launches_per_call * K), "parity": "bit-exact vs oracle/pileup_oracle.c on the first 65536 columns of the bench input",
            "config": {"workload": "pileup feature counting (calculate_clair3_pileup) over a synthetic %d-column region, mean depth %d, "
                                   "%d reads of ~%d bases (%d CIGAR words), %d aligned bases, %d candidates; %d calls in flight"
                                   % (cfg["region"], cfg["depth"], host.n_reads, cfg["read_len"], len(host.cigar), bases, n_cand, n_ctr)},
-           "e2e": {"value": e2e_value, "unit": "bases/s", "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": d2h, "steps": max(2, K // 4),
-                   "repeats": re["repeats"], "timed_region_s": re["ms"] * 1e-3,
+           "e2e": {"value": e2e_value, "unit": "bases/s", "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": d2h, "steps": K,
+                   "timed_region_s": e2e_ms * 1e-3,
                    "mode": "PileupCounter.count(pinned host records).fetch(pinned=True): H2D of the records, 8 kernels, D2H of matrix / major / stats / candidates into page-locked buffers, synchronous per call"},
            "roofline": {"bound": "hbm", "achieved": ach, "peak": pk["hbm"], "unit": "GB/s", "frac": ach / pk["hbm"], "traffic": traffic,
                         "peak_source": pk["which"], "kernel": "all 8 kernels of one call, timed alone with CUDA events on its stream (c3b_plp_last_ms): %.3f ms" % ms_alone,
@@ -856,7 +871,7 @@ def select_workloads(spec, explicit, world):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20, help="K: steps per repeat (every timed region repeats the K steps until it lasts >= 2 s)")
+    ap.add_argument("--steps", type=int, default=20, help="K: steps in every timed region")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workloads", default="pileup,fa,fa_dwell,cascade,pileup_counts")
@@ -868,15 +883,15 @@ def main():
                          "smallest GPU-filling tile for synchronous host-buffer calls)")
     ap.add_argument("--opt", action="append", default=[], help="library option name=value for the pileup model (tuning runs), repeatable")
     ap.add_argument("--no-cpu-baseline", action="store_true")
-    ap.add_argument("--min-region-s", type=float, default=2.0,
-                    help="minimum length of every timed region (profiling runs under ncu pass 0: one pass of the K steps)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs of every workload as DIR/<name>.npy (b200 arm, rank 0)")
     args = ap.parse_args()
     explicit = args.workload is not None or any(a.startswith("--workloads") for a in sys.argv[1:])
     args.workloads = select_workloads(args.workload or args.workloads, explicit, int(os.environ.get("WORLD_SIZE", "1")))
-    global MIN_REGION_S
-    MIN_REGION_S = max(0.0, args.min_region_s)
     if args.steps <= 0:
-        args.steps = 20
+        ap.error("--steps must be >= 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs records the b200 arm's outputs")
     requested_warmup = args.warmup
     if args.warmup < 3:
         args.warmup = 3                                               # the timing rules ask for >= 3 warm-up steps
@@ -965,7 +980,7 @@ def main():
         line = {
             "metric": "candidate-sites/sec", "value": head["value"], "unit": "sites/s", "n_gpus": world, "steps": args.steps,
             "warmup": requested_warmup, "warmup_steps_run": args.warmup, "ms_per_step": head.get("ms_per_step", head.get("ms_per_pass")),
-            "repeats": head["repeats"], "timed_region_s": head["timed_region_s"],
+            "timed_region_s": head["timed_region_s"],
             "higher_is_better": True, "scaling": head["scaling"], "vs_baseline": None, "dtype": "f16", "data": "synthetic",
             "config": head["config"], "run": head.get("run"),
             "clocks": head["clocks"],
@@ -978,6 +993,8 @@ def main():
             "weight_broadcast": bcast,
             "workloads": subs,
         }
+        if ctx.dump is not None:
+            dump_outputs(args.dump_outputs, ctx.dump)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()

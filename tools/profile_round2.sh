@@ -1,10 +1,10 @@
 #!/bin/bash
 # Round-2 ncu evidence (run under gpurun, one GPU): launch lists (kernel shares) and one `--set full` capture of every distinct
-# kernel of both networks, single stream, no 2-s regions (--min-region-s 0).  Outputs -> gpurun_out/${R}_*.
+# kernel of both networks, single stream, every timed region exactly the K steps.
 set -u
 R=${1:-r2p}
 mkdir -p gpurun_out
-B="python bench.py --steps 4 --warmup 3 --no-cpu-baseline --min-region-s 0 --streams 1"
+B="python bench.py --steps 4 --warmup 3 --no-cpu-baseline --streams 1"
 timeout 400 ncu --metrics gpu__time_duration.sum --clock-control none -c 400 --csv --log-file gpurun_out/${R}_launches_pileup.csv \
     $B --workloads pileup > gpurun_out/${R}_ncu_launch_p.log 2>&1
 timeout 400 ncu --metrics gpu__time_duration.sum --clock-control none -c 800 --csv --log-file gpurun_out/${R}_launches_fa.csv \

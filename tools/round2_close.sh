@@ -19,7 +19,7 @@ timeout -k 10 120 ncu --metrics gpu__time_duration.sum --clock-control none -c 4
     python tools/plp_diag.py prof 1048576 3 > gpurun_out/${R}_ncu_launch_plp.log 2>&1
 timeout -k 10 180 ncu --set full --clock-control none --import-source on -k regex:"plp_count_tile" -s 1 -c 1 \
     -o gpurun_out/${R}_prof_plp python tools/plp_diag.py prof 1048576 3 > gpurun_out/${R}_ncu_full_plp.log 2>&1
-B="python bench.py --steps 4 --warmup 3 --no-cpu-baseline --min-region-s 0 --streams 1"
+B="python bench.py --steps 4 --warmup 3 --no-cpu-baseline --streams 1"
 timeout -k 10 200 ncu --metrics gpu__time_duration.sum --clock-control none -c 400 --csv --log-file gpurun_out/${R}_launches_pileup.csv \
     $B --workloads pileup > gpurun_out/${R}_ncu_launch_p.log 2>&1
 timeout -k 10 300 ncu --set full --clock-control none --import-source on -k regex:"lstm_tc_kernel|lstm_pair_kernel|lstm2x|proj2_kernel|tail_kernel|ingest_pileup" -s 20 -c 5 \

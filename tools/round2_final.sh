@@ -21,7 +21,7 @@ for tool in memcheck racecheck synccheck; do
   timeout -k 10 300 $SAN --tool $tool --print-limit 5 python tools/sanitize_case.py f 16 pconv_impl=1 > gpurun_out/${R}_san_fa2_${tool}.log 2>&1
   echo "$tool [full-alignment, pconv_impl=1 (CTA pairs)] :: $(grep -E 'ERROR SUMMARY|RACECHECK SUMMARY|ok \(' gpurun_out/${R}_san_fa2_${tool}.log | tr '\n' ' ')"
 done
-B="python bench.py --steps 4 --warmup 3 --no-cpu-baseline --min-region-s 0 --streams 1"
+B="python bench.py --steps 4 --warmup 3 --no-cpu-baseline --streams 1"
 timeout -k 10 400 ncu --metrics gpu__time_duration.sum --clock-control none -c 400 --csv --log-file gpurun_out/${R}_launches_pileup.csv \
     $B --workloads pileup > gpurun_out/${R}_ncu_launch_p.log 2>&1
 timeout -k 10 600 ncu --set full --clock-control none --import-source on -k regex:"lstm_tc_kernel|lstm_pair_kernel|proj2_kernel|tail_kernel|ingest_pileup" -s 20 -c 5 \
