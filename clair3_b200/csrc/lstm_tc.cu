@@ -17,7 +17,7 @@
 //
 // LSTM1 (H=128): K = 48 + 128.  The 48 x columns are [hi(x) (18) | 1 | lo(x) (18) | 0...]: the raw counts are unbounded integers
 // (the reference's GPU branch does not rescale depth, clair3/CallVariantsFromCffi.py:299-353), fp16 is exact only to 2048, so
-// every count is split as x = hi + lo with hi = fp16(x) and lo = fp16(x - hi) - exact for |x| <= 131 008, saturating beyond -
+// every count is split as x = hi + lo with hi = fp16(x) and lo = fp16(x - hi) - exact for |x| <= 67 552 (hi stops at 65 504) -
 // and W_ih multiplies both parts (fp32 accumulate: the same result as an exact-input product).  Column 18 is a constant 1 that
 // carries b_ih + b_hh, so the x projection and the bias are fused into the same MMAs.  
 // LSTM2 (H=160, input 256): the input projection W_ih*h1 (+bias) is a separate big GEMM
@@ -447,7 +447,7 @@ __device__ __forceinline__ float ingest_to_float(T v) { return (float)v; }
 // Dense [batch][33][channels] tensor, or (starts != nullptr) 33-row windows of the per-column count matrix [n_cols][channels]
 // (libclair3's plp_data.matrix; preprocess/CreateTensorPileupFromCffi.py:362-394 slices the same windows on the host, zero
 // rows where a window overhangs the matrix) -> xs[t][bp][48] fp16 with columns [hi(x) | 1 | lo(x) | 0..]: hi = fp16(x)
-// (saturating at +-65504), lo = fp16(x - hi), so hi + lo == x exactly for |x| <= 131 008; column `channels` = constant 1
+// (saturating at +-65504), lo = fp16(x - hi), so hi + lo == x exactly for |x| <= 67 552; column `channels` = constant 1
 // (LSTM1's bias column).
 // tiled = 0: xs[t][bp][48] (lstm_tc_kernel); tiled = 1: xs2[t][bp/128][6 k-groups][128 sites][8] (the CTA-pair kernel bulk-copies one
 // 12 KB run per step and 128-site tile)

@@ -142,7 +142,7 @@ def test_pair_lstm1_kernel_full_size_deep_and_ragged():
     y = m(torch.from_numpy(x).cuda()).cpu().numpy()
     _assert_tol(_stats("pileup_1024_pair_lstm12", y, orc.pileup_forward(sd, x, False)))
     for n in (1, 129, 300, 1000):
-        assert np.abs(m(torch.from_numpy(x[:n]).cuda()).cpu().numpy() - y[:n]).max() < 1e-5
+        assert np.array_equal(m(torch.from_numpy(x[:n]).cuda()).cpu().numpy(), y[:n])
     xs = (x.astype(np.int64) * 75)
     xs[::2] = x[::2]
     xs = xs.astype(np.int32)
@@ -155,7 +155,7 @@ def test_pair_lstm1_kernel_full_size_deep_and_ragged():
     from oracle import decode_oracle as dec
     xw = dec.pileup_windows(cols, starts).astype(np.int32)
     yw = m.forward_windows(cols, starts).numpy()
-    assert np.abs(yw - m(torch.from_numpy(xw).cuda()).cpu().numpy()).max() < 1e-5
+    assert np.array_equal(yw, m(torch.from_numpy(xw).cuda()).cpu().numpy())
 
 
 @pytest.mark.parametrize("tile", [16, 32])
@@ -182,7 +182,7 @@ def test_pair_lstm2_kernel_full_size_and_streams():
     _assert_tol(_stats("pileup_1024_pair_lstm2", y, orc.pileup_forward(sd, x, False)))
     # ragged batches (odd number of 128-site tiles: the second CTA of the last pair works on padding) and stream consistency
     for n in (1, 129, 300, 1000):
-        assert np.abs(m(torch.from_numpy(x[:n]).cuda()).cpu().numpy() - y[:n]).max() < 1e-5
+        assert np.array_equal(m(torch.from_numpy(x[:n]).cuda()).cpu().numpy(), y[:n])
     xd = [torch.from_numpy(synth.pileup_inputs(1024, seed=300 + i)).cuda() for i in range(8)]
     ref = [m(v).cpu().numpy() for v in xd]
     streams = [torch.cuda.Stream() for _ in range(8)]
@@ -193,7 +193,7 @@ def test_pair_lstm2_kernel_full_size_and_streams():
                 outs[i] = m(xd[i])
         torch.cuda.synchronize()
         for i in range(8):
-            assert np.abs(outs[i].cpu().numpy() - ref[i]).max() < 1e-4
+            assert np.array_equal(outs[i].cpu().numpy(), ref[i])
 
 
 # ---------------------------------------------------------------------------------------------- deep sites, depth rescale
@@ -365,7 +365,7 @@ def test_forward_windows_equals_host_sliced_tensors(dtype):
     y_dense = m(torch.from_numpy(x).cuda()).cpu().numpy()
     y_win_dev = m.forward_windows(torch.from_numpy(cols).cuda(), torch.from_numpy(starts).cuda()).cpu().numpy()
     y_win_host = m.forward_windows(cols, starts).numpy()
-    assert np.abs(y_win_dev - y_dense).max() < 1e-5 and np.abs(y_win_host - y_dense).max() < 1e-5
+    assert np.array_equal(y_win_dev, y_dense) and np.array_equal(y_win_host, y_dense)
     from oracle import clair3_oracle as orc
     _assert_tol(_stats("forward_windows_%s" % np.dtype(dtype).name, y_win_dev[:256], orc.pileup_forward(sd, x[:256], False)), agree=0.98)
     m32 = _pileup(sd, precision=1)
@@ -384,13 +384,13 @@ def test_predict_stream_yields_in_order_and_matches_sync():
     got = list(m.predict_stream(iter(xs), streams=4))
     assert len(got) == len(want)
     for g, w in zip(got, want):
-        assert g.shape == w.shape and (g.size == 0 or np.abs(g - w).max() < 1e-5)
+        assert g.shape == w.shape and np.array_equal(g, w)
     sdf = synth.fa_state_dict(True, channels=8, seed=62)
     f = _fa(sdf)
     xf = [synth.fa_inputs(n, depth=89, channels=8, seed=80 + i) for i, n in enumerate([200, 256, 7, 256, 100])]
     wantf = [f(torch.from_numpy(x)).numpy() for x in xf]
     for g, w in zip(f.predict_stream(iter(xf), streams=3), wantf):
-        assert np.abs(g - w).max() < 1e-5
+        assert np.array_equal(g, w)
 
 
 # ---------------------------------------------------------------------------------------------- pconv_impl = 1
@@ -425,7 +425,7 @@ def test_pair_convolutions_full_size_ragged_and_streams():
     _assert_tol(_stats("pair_conv_300", y1, ref))
     assert np.abs(y1 - y0).max() < 5e-3            # same fp16 operands, different fp32 accumulation order (taps by parity plane)
     for n in (1, 3, 44, 129, 256, 257):
-        assert np.abs(m1(xd[:n]).cpu().numpy() - y1[:n]).max() < 1e-5, n
+        assert np.array_equal(m1(xd[:n]).cpu().numpy(), y1[:n]), n
     streams = [torch.cuda.Stream() for _ in range(6)]
     xs = [xd[: (256 if i % 2 else 77)] for i in range(6)]
     for rep in range(3):
@@ -435,7 +435,7 @@ def test_pair_convolutions_full_size_ragged_and_streams():
                 outs[i] = m1(xs[i])
         torch.cuda.synchronize()
         for i in range(6):
-            assert np.abs(outs[i].cpu().numpy() - y1[: xs[i].shape[0]]).max() < 1e-4
+            assert np.array_equal(outs[i].cpu().numpy(), y1[: xs[i].shape[0]])
 
 
 # ---------------------------------------------------------------------------------------------- full-alignment edges
@@ -450,12 +450,12 @@ def test_full_alignment_ragged_chunks_and_alternating_batches():
     y = m(xd).cpu().numpy()
     ya = m(xd[:256]).cpu().numpy()
     yb = m(xd[256:]).cpu().numpy()
-    assert np.abs(y[:256] - ya).max() < 1e-5 and np.abs(y[256:] - yb).max() < 1e-5
+    assert np.array_equal(y[:256], ya) and np.array_equal(y[256:], yb)
     x55 = synth.fa_inputs(40, depth=55, channels=8, seed=72)
     y55 = m(torch.from_numpy(x55).cuda()).cpu().numpy()
     for n in (44, 256, 3, 300, 129):
-        assert np.abs(m(xd[:n]).cpu().numpy() - y[:n]).max() < 1e-5
-        assert np.abs(m(torch.from_numpy(x55).cuda()).cpu().numpy() - y55).max() < 1e-5
+        assert np.array_equal(m(xd[:n]).cpu().numpy(), y[:n])
+        assert np.array_equal(m(torch.from_numpy(x55).cuda()).cpu().numpy(), y55)
 
 
 def test_full_alignment_concurrent_streams_are_consistent():
@@ -472,7 +472,7 @@ def test_full_alignment_concurrent_streams_are_consistent():
                 outs[i] = m(xd[i])
         torch.cuda.synchronize()
         for i in range(8):
-            assert np.abs(outs[i].cpu().numpy() - ref[i]).max() < 1e-4
+            assert np.array_equal(outs[i].cpu().numpy(), ref[i])
 
 
 def test_two_models_on_two_host_threads():
@@ -494,7 +494,7 @@ def test_two_models_on_two_host_threads():
                 with torch.cuda.stream(st):
                     y = model(x)
                 st.synchronize()
-                assert np.abs(y.cpu().numpy() - ref).max() < 1e-4
+                assert np.array_equal(y.cpu().numpy(), ref)
                 assert model.tap(tapname).size > 0
         except Exception as e:      # noqa: BLE001
             errs.append(e)
